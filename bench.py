@@ -123,6 +123,7 @@ class ClockSampler:
         if self.proc is None:
             return {"sm_mhz": None, "sm_max_mhz": None, "reasons": ["nvidia-smi unavailable"]}
         self.proc.terminate()
+        self.proc.wait()
         sm = [float(r[0]) for r in self.rows if r and r[0].replace(".", "").isdigit()]
         mx = [float(r[1]) for r in self.rows if len(r) > 1 and r[1].replace(".", "").isdigit()]
         names = ["hw_slowdown", "hw_thermal_slowdown", "sw_thermal_slowdown", "sw_power_cap"]
@@ -307,6 +308,13 @@ def run_reference_arm(a):
     print(json.dumps(line), flush=True)
 
 
+def dump_outputs(out_dir, **arrays):
+    """<out_dir>/<name>.npy in float32, one file per output array"""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), t.detach().float().cpu().numpy())
+
+
 # ---------------------------------------------------------------- BASELINE configs[4]: the full pipeline of one subject per GPU
 PIPE_METRIC = "motion-frames/sec full pipeline (guide keyframes + body 1000 steps + face ddim500, T=600)"
 PIPE_SAMPLES = 16          # samples per subject (configs[4]: 4 subjects x 16 samples)
@@ -430,6 +438,8 @@ def run_pipeline(a):
         dist.all_reduce(dt, op=dist.ReduceOp.MAX)
     barrier()
     assert torch.isfinite(res).all() and res.shape[0] == B * world
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, sample=res)
     if rank == 0:
         ms = dt.item() * 1e3 / a.steps
         v = world * B * T / (ms / 1e3)
@@ -462,7 +472,9 @@ def main():
     ap.add_argument("--no-cfg", action="store_true",
                     help="secondary measurement (SURVEY 8d, config 2 'no-CFG variant'): the bare denoiser, one forward per step; "
                          "not the benchmark line")
-    ap.add_argument("--dump-out", default=None, help="debug only: save the result of the last timed loop as .npy")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned to its caller as DIR/<name>.npy (float32), so that two builds "
+                         "can be compared output for output: the inputs depend only on the arguments")
     ap.add_argument("--split-terms", type=int, default=None, help="0: exact-fp32 FFMA arm; 2 (pose default, fused chain kernels) | 3 (face default): split-bf16 tcgen05 arms")
     ap.add_argument("--workload", default="pose", choices=["pose", "face", "pipeline"],
                     help="pose = BASELINE configs[1] (the contract line); face = configs[3] (ddim500, g=10, 16 rows/GPU); pipeline = configs[4] "
@@ -470,6 +482,10 @@ def main():
     ap.add_argument("--no-config3", action="store_true", help="skip the extra global-batch-32 (configs[2], strong-scaling) measurement")
     ap.add_argument("--no-gpu-baseline", action="store_true", help="skip the reference-on-this-GPU leg")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl == "reference":
+        ap.error("--dump-outputs: the reference arm times single diffusion steps, not whole loops")
     face = a.workload == "face"
     SPLIT_TERMS = a.split_terms if a.split_terms is not None else (3 if face else 2)
     if a.impl == "reference":
@@ -567,11 +583,13 @@ def main():
     launches0 = model.launch_count()
     clocks = ClockSampler(local)
     clocks.start()
-    ms_step, out = timed(loop_resident, a.steps)
-    clk = clocks.stop()
+    try:
+        ms_step, out = timed(loop_resident, a.steps)
+    finally:
+        clk = clocks.stop()
     launches = (model.launch_count() - launches0)
-    if a.dump_out and rank == 0:
-        np.save(a.dump_out, out.float().cpu().numpy())
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, sample=out)
     loop_e2e()
     ms_e2e, out_h = timed(loop_e2e, a.steps)
     assert out.shape[0] == B * world and torch.isfinite(out).all()

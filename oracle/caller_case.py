@@ -72,3 +72,44 @@ def inv_transform(data, data_type: str):
     """stand-in for Social.inv_transform (data_loaders/data.py:71-91): de-normalise with fixed synthetic statistics"""
     std, mean = {"pose": (0.5, 0.1), "face": (0.7, -0.2), "audio": (2.0, 0.3)}[data_type]
     return data * std + mean
+
+
+def caller_modules() -> dict:
+    """{import name: module} standing in for the reference checkout on sys.path: the module attributes
+    `patch_reference()` swaps (the originals raise, so an unswapped one is caught) and a caller that makes the calls of
+    sample/generate.py `_setup_model` and `_run_single_diffusion` (:74-107, :252-268) with the same arguments, looking
+    the factories up in its module at call time as the original does, plus the stand-in fairseq the model's
+    constructor loads the frozen extractor through (model/utils.py:18-26)."""
+    import types
+
+    from oracle.ref_harness import fairseq_standin_modules
+
+    def unswapped(*a, **k):
+        raise AssertionError("patch_reference() left the reference's own factory in place")
+    mods = {n: types.ModuleType(n) for n in ("utils", "utils.model_util", "model", "model.cfg_sampler", "sample", "sample.generate")}
+    mu, cs, gen = mods["utils.model_util"], mods["model.cfg_sampler"], mods["sample.generate"]
+    mu.create_model_and_diffusion = mu.load_model = mu.create_gaussian_diffusion = unswapped
+    cs.ClassifierFreeSampleModel = gen.ClassifierFreeSampleModel = unswapped
+    gen.create_model_and_diffusion = gen.load_model = unswapped
+    mods["utils"].model_util, mods["model"].cfg_sampler, mods["sample"].generate = mu, cs, gen
+
+    def _setup_model(args):
+        model, diffusion = gen.create_model_and_diffusion(args, split_type="test")
+        gen.load_model(model, torch.load(args.model_path, map_location="cpu"))
+        if args.guidance_param != 1:
+            model = gen.ClassifierFreeSampleModel(model)
+        model.to(args.device)
+        model.eval()
+        return model, diffusion
+
+    def _run_single_diffusion(args, model_kwargs, diffusion, model, inv_transform, gt):
+        with torch.no_grad():
+            sample = diffusion.ddim_sample_loop(model, (args.batch_size, model.nfeats, 1, args.curr_seq_length), clip_denoised=False,
+                                                model_kwargs=model_kwargs, init_image=None, progress=True, dump_steps=None,
+                                                noise=None, const_noise=False)
+        to_frames = lambda t: inv_transform(t.cpu().permute(0, 2, 3, 1), args.data_format).permute(0, 3, 1, 2)
+        return (to_frames(sample), inv_transform(model_kwargs["y"]["audio"].cpu().numpy(), "audio"),
+                inv_transform(model_kwargs["y"]["keyframes"], args.data_format), to_frames(gt))
+    gen._setup_model, gen._run_single_diffusion = _setup_model, _run_single_diffusion
+    mods.update(fairseq_standin_modules())
+    return mods

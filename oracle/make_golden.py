@@ -228,10 +228,51 @@ def golden_caller():
     print("caller_pose.npz written", tuple(sample.shape), float(sample.abs().max()))
 
 
+def golden_guide():
+    """The reference's GuideTransformer (logits + KV-free generate under an inverse-CDF draw) and TemporalVertexCodec.decode
+    with the seeded weights of oracle/guide_case.py -> tests/golden/guide.npz."""
+    from torch.distributions import Categorical
+    from oracle import guide_case as GC
+    ref = RH.import_reference()
+    import model.guide as G
+    import model.vqvae as V
+    c = GC.GUIDE
+    with RH._cwd(ref.scratch):
+        m = G.GuideTransformer(tokens=c["tokens"], num_layers=c["layers"], dim=c["dim"], emb_len=798, num_audio_layers=2).eval()
+    fixed = {k: m.state_dict()[k].clone() for k in ("rotary.freqs", "audio_resampler.kernel")}
+    guide_layout = GC.layout(m.state_dict())
+    m.load_state_dict(GC.seeded_state(guide_layout, c["seed"], fixed), strict=True)
+    B = c["B"]
+    cond = GC.guide_audio(B)
+    with torch.no_grad():
+        logits = m(GC.guide_tokens(B, c["n"], c["tokens"]), cond)
+    draw = GC.inverse_cdf_draw(GC.uniform_tape(B))
+    old = Categorical.sample
+    Categorical.sample = lambda self, *a, **k: draw(self.probs)
+    try:
+        tokens = m.generate(cond, sequence_length=4, layers=3, n_sequences=B)
+    finally:
+        Categorical.sample = old
+    v = GC.VQ
+    codec = V.TemporalVertexCodec(n_vertices=v["n_vertices"], latent_dim=v["latent_dim"], categories=v["categories"],
+                                  residual_depth=v["residual_depth"]).eval()
+    vq_layout = GC.layout(codec.state_dict())
+    codec.load_state_dict(GC.seeded_state(vq_layout, v["seed"]), strict=True)
+    with torch.no_grad():
+        decoded = codec.decode(GC.vq_codes())
+    np.savez_compressed(os.path.join(GOLD, "guide.npz"), guide_layout=guide_layout, guide_fixed_freqs=fixed["rotary.freqs"].numpy(),
+                        guide_fixed_kernel=fixed["audio_resampler.kernel"].numpy(), logits=logits.numpy(), tokens=tokens.numpy(),
+                        vq_layout=vq_layout, vq_decoded=decoded.numpy())
+    print("guide.npz written", tuple(logits.shape), tuple(tokens.shape), tuple(decoded.shape))
+
+
 def main():
     torch.manual_seed(0)
     torch.set_num_threads(8)
     os.makedirs(GOLD, exist_ok=True)
+    if "guide" in sys.argv:
+        golden_guide()
+        return
     if "plms" in sys.argv:
         golden_plms()
         return

@@ -70,9 +70,8 @@ class _StandInWav2Vec(nn.Module):
         self.feature_aggregator = nn.Conv1d(512, 512, 1)
 
 
-def _install_fairseq_standin() -> None:
-    if "fairseq" in sys.modules:
-        return
+def fairseq_standin_modules() -> dict:
+    """{import name: module} of the stand-in `fairseq` (shim 1)"""
     fs = types.ModuleType("fairseq")
     cu = types.ModuleType("fairseq.checkpoint_utils")
 
@@ -82,8 +81,13 @@ def _install_fairseq_standin() -> None:
 
     cu.load_model_ensemble_and_task = load_model_ensemble_and_task
     fs.checkpoint_utils = cu
-    sys.modules["fairseq"] = fs
-    sys.modules["fairseq.checkpoint_utils"] = cu
+    return {"fairseq": fs, "fairseq.checkpoint_utils": cu}
+
+
+def _install_fairseq_standin() -> None:
+    if "fairseq" in sys.modules:
+        return
+    sys.modules.update(fairseq_standin_modules())
 
 
 _scratch = None

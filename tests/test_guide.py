@@ -1,86 +1,55 @@
 """N2 / N3 (SURVEY 8f): the KV-cached guide sampler and the VQ decoder against the reference's own modules
 (model/guide.py GuideTransformer, model/vqvae.py TemporalVertexCodec) on CPU, with reference-layout checkpoints.
-Host-side PyTorch: no GPU needed.  Skipped when no reference view is importable."""
+tests/golden/guide.npz holds the reference's outputs for the seeded weights and inputs of oracle/guide_case.py
+(oracle/make_golden.py guide).  Host-side PyTorch: no GPU needed."""
 import json
 import os
 
 import numpy as np
-import pytest
 import torch
 
-from oracle import ref_harness as RH
-
-pytestmark = pytest.mark.skipif(not RH.reference_available(), reason="no reference view (python -m oracle.build_ref)")
-
-
-def _ref_guide(tokens=32, layers=2, dim=64):
-    ref = RH.import_reference()
-    import model.guide as G
-    torch.manual_seed(5)
-    with RH._cwd(ref.scratch):
-        m = G.GuideTransformer(tokens=tokens, num_layers=layers, dim=dim, emb_len=798, num_audio_layers=2).eval()
-    for p in m.parameters():                       # non-trivial biases / affine so every term is exercised
-        if p.dim() == 1:
-            torch.nn.init.normal_(p, 0.0 if "bias" in "" else 0.0, 0.05)
-    return m
+from oracle import guide_case as GC
+from oracle.ref_harness import _StandInWav2Vec
 
 
-def _audio(B, frames=240, seed=3):
-    g = torch.Generator().manual_seed(seed)
-    return 0.1 * torch.randn(B, frames * 1600, 2, generator=g)
+def _golden(golden_dir):
+    return np.load(os.path.join(golden_dir, "guide.npz"))
 
 
-def test_guide_sampler_logits_and_generate_match_reference():
+def test_guide_sampler_logits_and_generate_match_reference(golden_dir):
     from audio2photoreal_b200.guide import GuideSampler
-    m = _ref_guide()
-    ours = GuideSampler(m.state_dict(), tokens=m.tokens, audio_model=m.audio_model).eval()
-    assert set(ours.state_dict()) == set(m.state_dict())          # same checkpoint layout, frozen extractor included
-    B, n = 2, 12
-    cond = _audio(B)
-    g = torch.Generator().manual_seed(9)
-    toks = torch.cat([torch.full((B, 1), m.tokens), torch.randint(0, m.tokens, (B, n - 1), generator=g)], dim=1)
-    with torch.no_grad():
-        ref_logits = m(toks, cond)
-    got = ours.logits_for(toks, cond)
+    g, c = _golden(golden_dir), GC.GUIDE
+    layout = str(g["guide_layout"])
+    sd = GC.seeded_state(layout, c["seed"], {"rotary.freqs": g["guide_fixed_freqs"], "audio_resampler.kernel": g["guide_fixed_kernel"]})
+    audio_model = _StandInWav2Vec(large=False).eval()            # the frozen extractor the reference's constructor loads
+    audio_model.load_state_dict({k[len("audio_model."):]: v for k, v in sd.items() if k.startswith("audio_model.")})
+    ours = GuideSampler(sd, tokens=c["tokens"], audio_model=audio_model).eval()
+    assert set(ours.state_dict()) == {k for k, _, _ in json.loads(layout)}     # same checkpoint layout, frozen extractor included
+    B = c["B"]
+    cond = GC.guide_audio(B)
+    ref_logits = torch.from_numpy(g["logits"])
+    got = ours.logits_for(GC.guide_tokens(B, c["n"], c["tokens"]), cond)
     assert torch.allclose(got, ref_logits, rtol=1e-4, atol=2e-5), (got - ref_logits).abs().max().item()
 
     # generate(): identical token sequences under the same uniform tape (inverse-CDF draw on both sides)
-    tape = torch.rand(64, B, generator=torch.Generator().manual_seed(11))
-
-    def make_draw():
-        it = iter(tape)
-        return lambda probs: (torch.cumsum(probs, -1) < next(it).unsqueeze(-1)).sum(-1).clamp(max=probs.shape[-1] - 1)
-    from torch.distributions import Categorical
-    d_ref = make_draw()
-    old = Categorical.sample
-    Categorical.sample = lambda self, *a, **k: d_ref(self.probs)
-    try:
-        ref_tok = m.generate(cond, sequence_length=4, layers=3, n_sequences=B)
-    finally:
-        Categorical.sample = old
-    got_tok = ours.generate(cond, sequence_length=4, layers=3, n_sequences=B, draw=make_draw())
+    got_tok = ours.generate(cond, sequence_length=4, layers=3, n_sequences=B, draw=GC.inverse_cdf_draw(GC.uniform_tape(B)))
+    ref_tok = torch.from_numpy(g["tokens"])
     assert got_tok.shape == ref_tok.shape == (B, 12) and torch.equal(got_tok, ref_tok)
 
 
-def test_vq_decoder_matches_reference_and_checkpoint_layout(tmp_path):
+def test_vq_decoder_matches_reference_and_checkpoint_layout(golden_dir, tmp_path):
     from audio2photoreal_b200.guide import VQDecoder, setup_tokenizer
-    RH.import_reference()
-    import model.vqvae as V
-    torch.manual_seed(2)
-    codec = V.TemporalVertexCodec(n_vertices=104, latent_dim=64, categories=32, residual_depth=4).eval()
-    for layer in codec.quantizer.layers:
-        layer._codebook.embed.normal_()            # kmeans_init leaves zeros until training
+    g, v = _golden(golden_dir), GC.VQ
     d = tmp_path / "vq"
     d.mkdir()
     with open(d / "args.json", "w") as f:
-        json.dump({"nb_joints": 104, "output_emb_width": 64, "code_dim": 32, "depth": 4}, f)
-    torch.save({"net": codec.state_dict()}, d / "net_iter.pth")
+        json.dump({"nb_joints": v["n_vertices"], "output_emb_width": v["latent_dim"], "code_dim": v["categories"],
+                   "depth": v["residual_depth"]}, f)
+    torch.save({"net": GC.seeded_state(str(g["vq_layout"]), v["seed"])}, d / "net_iter.pth")
     ours = setup_tokenizer(str(d / "net_iter.pth"), device="cpu")
     assert isinstance(ours, VQDecoder) and ours.residual_depth == 4 and ours.n_clusters == 32
-    q = torch.randint(0, 32, (3, 20, 4))
-    with torch.no_grad():
-        want = codec.decode(q)
-    got = ours.decode(q)
+    want = torch.from_numpy(g["vq_decoded"])
+    got = ours.decode(GC.vq_codes())
     assert got.shape == want.shape == (3, 20, 104)
     assert torch.allclose(got, want, rtol=1e-5, atol=1e-6)
 

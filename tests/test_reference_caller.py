@@ -1,21 +1,20 @@
-"""The unchanged caller: the reference's own `sample/generate.py` functions `_setup_model` and `_run_single_diffusion`
-(sample/generate.py:74-97,252-268) driven through `audio2photoreal_b200.api.patch_reference()` with RAW y["audio"].
+"""The caller: what the reference's `sample/generate.py` functions `_setup_model` and `_run_single_diffusion`
+(sample/generate.py:74-97,252-268) do, driven through `audio2photoreal_b200.api.patch_reference()` with RAW y["audio"].
 
-The caller's source is imported from the reference checkout (in the build container) or from oracle/_ref, the byte-for-byte
-view oracle/build_ref.py writes (git-ignored, travels to the GPU box).  fairseq is not installed anywhere, so the frozen
-vq-wav2vec is ref_harness's stand-in conv stack, loaded through `fairseq.checkpoint_utils` exactly where the reference's
-constructor loads it (model/diffusion.py:140,270-271; model/utils.py:18-26).  The golden output comes from the UNPATCHED
-reference run on CPU (oracle/make_golden.py caller)."""
+oracle/caller_case.py stands in for the reference checkout under its import names (utils.model_util, model.cfg_sampler,
+sample.generate): a caller that makes the same calls with the same arguments, looking up the factories patch_reference()
+swaps.  fairseq is not installed anywhere, so the frozen vq-wav2vec is ref_harness's stand-in conv stack, loaded through
+`fairseq.checkpoint_utils` exactly where the reference's constructor loads it (model/diffusion.py:140,270-271;
+model/utils.py:18-26).  The golden output comes from the UNPATCHED reference's own caller run on CPU
+(oracle/make_golden.py caller)."""
 import os
+import sys
 
 import numpy as np
 import pytest
 import torch
 
 from oracle import caller_case as CC
-from oracle import ref_harness as RH
-
-needs_ref = pytest.mark.skipif(not RH.reference_available(), reason="no reference view (run python -m oracle.build_ref)")
 
 
 @pytest.fixture(autouse=True)
@@ -25,27 +24,26 @@ def _restore_reference_modules():
     unpatch_reference()
 
 
-def _patched_generate():
-    ref = RH.import_reference()                 # reference root on sys.path + fairseq stand-in + scratch cwd with assets/
-    import sample.generate as gen
+def _patched_generate(monkeypatch, cwd):
+    for name, mod in CC.caller_modules().items():
+        monkeypatch.setitem(sys.modules, name, mod)
+    monkeypatch.chdir(cwd)                      # the constructor resolves ./assets/ against the working directory
     from audio2photoreal_b200.api import patch_reference
     patch_reference()
-    return ref, gen
+    return sys.modules["sample.generate"]
 
 
-@needs_ref
-def test_setup_model_builds_the_b200_objects_and_fails_loudly_without_gpu(tmp_path):
+def test_setup_model_builds_the_b200_objects_and_fails_loudly_without_gpu(tmp_path, monkeypatch):
     """host side of the drop-in (no GPU needed): the caller's own `_setup_model` constructs Denoiser / CFGDenoiser / Sampler,
     the constructor sets up the frozen extractor like the reference's, a real-layout checkpoint (with audio_model.*) loads,
     and sampling on a CPU device raises instead of falling back."""
     from audio2photoreal_b200 import _lib
     from audio2photoreal_b200.api import CFGDenoiser, Denoiser, Sampler
-    ref, gen = _patched_generate()
+    gen = _patched_generate(monkeypatch, tmp_path)
     path = str(tmp_path / "model000000.pt")
     CC.write_checkpoint(path)
     args = CC.caller_args(path, "cpu")
-    with RH._cwd(ref.scratch):
-        model, diffusion = gen._setup_model(args)
+    model, diffusion = gen._setup_model(args)
     assert isinstance(model, CFGDenoiser) and isinstance(model.model, Denoiser) and isinstance(diffusion, Sampler)
     assert model.model.audio_model is not None and not model.training
     want = CC.standin_audio_state()
@@ -57,11 +55,10 @@ def test_setup_model_builds_the_b200_objects_and_fails_loudly_without_gpu(tmp_pa
         gen._run_single_diffusion(args, mk, diffusion, model, CC.inv_transform, gt)
 
 
-@needs_ref
 @pytest.mark.gpu
 @pytest.mark.parametrize("terms", [0, 2])
 def test_unchanged_caller_with_raw_audio_vs_reference_golden(golden_dir, tmp_path, monkeypatch, terms):
-    ref, gen = _patched_generate()
+    gen = _patched_generate(monkeypatch, tmp_path)
     monkeypatch.setenv("A2P_SPLIT_TERMS", str(terms))
     torch.backends.cudnn.allow_tf32 = False                    # the golden is CPU fp32: keep the frozen conv stack fp32 here too
     torch.backends.cuda.matmul.allow_tf32 = False
@@ -69,8 +66,7 @@ def test_unchanged_caller_with_raw_audio_vs_reference_golden(golden_dir, tmp_pat
     CC.write_checkpoint(path)
     args = CC.caller_args(path, "cuda:0")
     gt, mk = CC.caller_inputs()
-    with RH._cwd(ref.scratch):
-        model, diffusion = gen._setup_model(args)
+    model, diffusion = gen._setup_model(args)
     mk["y"] = {k: v.to(args.device) if torch.is_tensor(v) else v for k, v in mk["y"].items()}     # generate.py:131-134
     # the loop draws its initial noise with th.randn(*shape, device=device) (noise=None): CUDA and CPU generators differ, so the
     # test hands the loop the CPU draw the golden run used (test-side only; nothing else in the path is random at eta = 0)
